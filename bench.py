@@ -8,6 +8,7 @@ priority 1, pattern od, AS183-exact RNG. Every step mutates the NEXT window of c
 advances), so no step repeats work and the 6.5 GB corpus + 6.5 GB of outputs per step never fit L2.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3|c3num|c2|c4|c5] [--async-depth D]
+                  [--dump-outputs DIR]
 
 The default (C3) line also carries `parity_sample` (sampled case ids of the last timed step re-run through the oracle),
 `extra_workloads` (short C2 and C4 runs, value net of flagged cases, all-threads CPU port beside them) and, for c5, `collective`.
@@ -103,11 +104,17 @@ class ClockSampler:
         for ln in self.proc.stdout:
             self.lines.append((time.time(), ln.strip()))
 
+    def close(self):
+        """ends nvidia-smi whatever happened in between: no poller outlives the benchmark"""
+        if self.proc and self.proc.poll() is None:
+            self.proc.terminate()
+            self.proc.wait(10)
+
     def stop(self, t0=None, t1=None):
         if not self.proc:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
         time.sleep(0.06)
-        self.proc.terminate()
+        self.close()
         inside = [ln for (t, ln) in self.lines if t0 is not None and t0 <= t <= t1 + 0.03]
         window = "timed region"
         if not inside:      # a region shorter than the polling period: the samples right around it
@@ -153,7 +160,33 @@ def make_corpus_device(torch, kind, n, size, dev, seed):
     return data, off
 
 
-def measure(torch, dist, eng, args, workload, steps, warmup, rank, world, local, n_override=0, want_e2e=True, sampler=None):
+DUMP_BYTES = 12 << 20        # output bytes sampled by --dump-outputs: 48 MiB as float32, beside 8 bytes per case of lengths
+
+
+def dump_outputs(torch, out_dir, first_case, size, d_out, d_out_off, d_out_len, st):
+    """What the caller of the timed step received in the last step, as .npy files (float64 / float32) for comparing two builds:
+      out_len      every case's output length;
+      sample_case  the case ids of a fixed sample (seeded, independent of the outputs, so two builds sample the same cases);
+      sample_out   their output bytes, one row per sampled case, the first 2 x seed_bytes of each, -1 past the case's end;
+      stats        n_cases, bytes_in, bytes_out, n_unsupported, n_died, n_overflow of the step (eb200_stats without the timings)."""
+    import numpy as np
+    n = d_out_len.numel()
+    width = 2 * size
+    count = max(1, min(n, 4096, DUMP_BYTES // width))
+    ks = np.sort(np.random.Generator(np.random.PCG64(0xD0)).choice(n, size=count, replace=False))
+    kt = torch.from_numpy(ks).to(d_out.device)
+    col = torch.arange(width, dtype=torch.int64, device=d_out.device)
+    idx = d_out_off[kt][:, None] + col[None, :]
+    inside = col[None, :] < d_out_len[kt][:, None]
+    rows = torch.where(inside, d_out[idx.clamp(0, d_out.numel() - 1)].float(), torch.full_like(idx, -1, dtype=torch.float32))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "out_len.npy"), d_out_len.cpu().numpy().astype(np.float64))
+    np.save(os.path.join(out_dir, "sample_case.npy"), (first_case + ks).astype(np.float64))
+    np.save(os.path.join(out_dir, "sample_out.npy"), rows.cpu().numpy())
+    np.save(os.path.join(out_dir, "stats.npy"), np.array([st.n_cases, st.bytes_in, st.bytes_out, st.n_unsupported, st.n_died, st.n_overflow], dtype=np.float64))
+
+
+def measure(torch, dist, eng, args, workload, steps, warmup, rank, world, local, n_override=0, want_e2e=True, sampler=None, dump_dir=None):
     """W warm-up steps + K timed steps of one workload on this rank's GPU; returns the fields of the JSON line (rank 0) or None"""
     import erlamsa_b200
     from erlamsa_b200 import _native as N
@@ -241,6 +274,8 @@ def measure(torch, dist, eng, args, workload, steps, warmup, rank, world, local,
         ms = float(t[0].item()); nflag = int(t[1].item())
         dist.barrier()
     out_len_sum = int(d_out_len.sum().item())
+    if dump_dir and rank == 0:
+        dump_outputs(torch, dump_dir, 1 + (rank + world * (warmup + steps - 1)) * n_cases, size, d_out, d_out_off, d_out_len, st)
 
     # ---- parity sample: case ids of the LAST timed step, re-run through the oracle on the host (checker only, after the clock)
     parity = None
@@ -414,7 +449,11 @@ def run_ours(args):
     if rank == 0 and not os.environ.get("EB200_BENCH_NO_SAMPLER"):
         sampler.start()
         time.sleep(0.5)
-    line = measure(torch, dist, eng, args, args.workload, args.steps, args.warmup, rank, world, local, n_override=args.cases, sampler=sampler)
+    try:
+        line = measure(torch, dist, eng, args, args.workload, args.steps, args.warmup, rank, world, local, n_override=args.cases, sampler=sampler,
+                       dump_dir=args.dump_outputs)
+    finally:
+        sampler.close()
     if rank == 0 and not args.no_cpu:
         n_cases, size, kind, muts, pats, desc = WORKLOADS[args.workload]
         muts = {c: 1 for c in muts} if muts is not None else {c: p for c, p in erlamsa_b200.default_mutations() if c in erlamsa_b200.supported_mutations()}
@@ -543,7 +582,13 @@ def main():
     ap.add_argument("--e2e-cases", type=int, default=0, help="cases per e2e step (0 = the whole config)")
     ap.add_argument("--e2e-steps", type=int, default=2)
     ap.add_argument("--async-depth", type=int, default=0, help="also time the steps through eb200_submit_device / eb200_collect with this many batches in flight (0 = off)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (lengths, a fixed sample of output bytes, counters) as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

@@ -8,18 +8,23 @@ it calls (erlamsa_main, erlamsa_mutations, erlamsa_patterns, erlamsa_gen).
    the real NIF receives -- fuzz_batch/2 must return what the reference returns case by case, including a case the
    mock reports as {flagged, I, St, Why} (re-run alone through erlamsa_main:fuzzer/1) and empty results being dropped.
 
-Needs /root/reference (build container only); skipped elsewhere. CPU only."""
+The reference's sources are not part of this repository: what its modules answered to these tests is recorded in
+tests/golden/erlang_shim_calls.json and replayed (oracle/erlref/replay.py), so a call the project's Erlang makes with other
+arguments than when it was recorded fails. With the reference's sources present (ERLAMSA_REFERENCE_SRC),
+`ERLREF_RECORD=1 python -m pytest tests/test_erlang_shim.py` runs them there and rewrites the file. CPU only."""
 import os
 import sys
 
 import pytest
 
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "oracle"))
-from erlref import refrun  # noqa: E402
-
-pytestmark = pytest.mark.skipif(not refrun.available(), reason="the reference's sources are only in the build container")
+from erlref import refrun, replay  # noqa: E402
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+CALLS = replay.Calls(os.path.join(ROOT, "tests", "golden", "erlang_shim_calls.json"), record=bool(os.environ.get("ERLREF_RECORD")))
+if CALLS.record and not refrun.available():
+    raise RuntimeError("ERLREF_RECORD needs the reference's sources (ERLAMSA_REFERENCE_SRC)")
+
 SEED = (11, 22, 33)
 BLOBS = [b"hello 100 world 42\n", b"alpha beta\ngamma delta\nalpha beta\n", b"<a href=\"x\">t</a> 7 'q' 12345\n", bytes(range(64)) * 3]
 
@@ -34,11 +39,24 @@ def in_evaluator(fn):
     return box["v"]
 
 
+def reference(*extra_dirs):
+    """an evaluator with the project's Erlang modules loaded on demand and the reference's modules answered by CALLS"""
+    r = refrun.Reference()
+    r.rt.src_dirs.extend([os.path.join(ROOT, "erlang")] + list(extra_dirs))
+    CALLS.attach(r.rt, refrun.REF_SRC)
+    return r
+
+
+@pytest.fixture(scope="module", autouse=True)
+def recorded_calls():
+    yield CALLS
+    if CALLS.record:
+        CALLS.save()
+
+
 @pytest.fixture(scope="module")
 def ref():
-    r = refrun.Reference()
-    r.rt.src_dirs.append(os.path.join(ROOT, "erlang"))
-    return r
+    return reference()
 
 
 def call(ref, mod, fun, *args):
@@ -91,8 +109,7 @@ def test_without_the_nif_every_call_is_the_reference_with_the_callers_numbering(
 
 def test_with_a_mock_nif_the_gpu_branch_returns_what_the_reference_returns():
     import oracle_lib as O
-    ref = refrun.Reference()                                            # a fresh runtime: call sites cache their targets, the stub must never have run
-    ref.rt.src_dirs.append(os.path.join(ROOT, "erlang"))
+    ref = reference()                                                   # a fresh runtime: call sites cache their targets, the stub must never have run
     from erlref.interp import Bif
     from erlref.terms import from_py, to_py
     seen = {}
@@ -131,8 +148,7 @@ def test_faas_batch_endpoint_answers_what_the_reference_would_case_by_case():
     import json
     import oracle_lib as O
     from erlref.terms import from_py, to_py
-    ref = refrun.Reference()
-    ref.rt.src_dirs.append(os.path.join(ROOT, "erlang"))
+    ref = reference()
     sent = []
 
     def flat(x, out):
@@ -192,9 +208,8 @@ def test_otp_dump_tool_runs_and_reproduces_the_committed_vectors(tmp_path):
             lines.append('{"%s",%d,"%s",%d,{%d,%d,%d},%s,%s,[%s]}' % (v["name"], k, v["blobs"][(i - 1) % len(v["blobs"])], i, v["seed"][0], v["seed"][1], v["seed"][2],
                                                                      plist(v["mutations"]), plist(v["patterns"]), ",".join(extra)))
             want[(v["name"], k)] = (v["status"][k], v["digests"][k])
-    ref = refrun.Reference()
+    ref = reference(str(tmp_path))
     rt = ref.rt
-    rt.src_dirs.append(str(tmp_path))
     out = []
 
     def flat(x, acc):

@@ -73,6 +73,40 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert line["cpu_baseline"]["kind"] == "port" and line["e2e"]["h2d_bytes_per_step"] == 0
 
 
+def test_bench_dump_outputs_writes_the_last_steps_results(tmp_path):
+    """`bench.py --dump-outputs DIR` on host tensors standing in for the device buffers: every case's length, a fixed seeded
+    sample of whole cases' bytes (-1 past each case's end), the step's counters; float arrays, at most 64 MB in all"""
+    import glob
+    import os
+    import sys
+    import numpy as np
+    import torch
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    sys.path.insert(0, root)
+    import bench
+    from erlamsa_b200 import _native as N
+    size, n = 4096, 3000
+    r = np.random.Generator(np.random.PCG64(3))
+    lens = r.integers(0, 2 * size + 100, n)
+    offs = np.concatenate([[0], np.cumsum(lens)])
+    out = torch.from_numpy(r.integers(0, 256, int(offs[-1]) + 64, dtype=np.uint8))
+    st = N.Stats(n_cases=n, bytes_in=n * size, bytes_out=int(lens.sum()), n_unsupported=2, n_died=1, n_overflow=0)
+    for d in ("a", "b"):
+        bench.dump_outputs(torch, str(tmp_path / d), 1001, size, out, torch.from_numpy(offs), torch.from_numpy(lens), st)
+    files = sorted(os.path.basename(p) for p in glob.glob(str(tmp_path / "a" / "*.npy")))
+    assert files == ["out_len.npy", "sample_case.npy", "sample_out.npy", "stats.npy"]
+    got = {f[:-4]: np.load(str(tmp_path / "a" / f)) for f in files}
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+    assert sum(os.path.getsize(str(tmp_path / "a" / f)) for f in files) <= 64 << 20
+    assert all(np.array_equal(got[f[:-4]], np.load(str(tmp_path / "b" / f))) for f in files)
+    assert np.array_equal(got["out_len"], lens) and list(got["stats"]) == [n, n * size, lens.sum(), 2, 1, 0]
+    ks = got["sample_case"].astype(np.int64) - 1001
+    assert len(ks) == min(n, bench.DUMP_BYTES // (2 * size)) and len(set(ks)) == len(ks)
+    for k, row in zip(ks, got["sample_out"]):
+        m = min(lens[k], 2 * size)
+        assert np.array_equal(row[:m], out[offs[k]:offs[k] + m].numpy()) and (row[m:] == -1).all()
+
+
 def test_markup_corpus_shapes():
     """C4 documents: exact size, SGML ones tokenise as markup, JSON ones as a complete document (oracle-side check)"""
     import oracle_lib as O

@@ -1,75 +1,66 @@
 """The reference's multi-threaded mode (`workers` > 1 with a file output; src/erlamsa_main.erl:88-111,254-280) as the host mirror plans it
 (erlamsa_b200/workers.py) and as the engine's host code seeds it (eb200_opts.case_stream_*), on the CPU:
-  * threading_mode/3 == the reference's get_threading_mode/3, executed from its source, for every (n, workers) up to (40, 9);
+  * threading_mode/3 == the reference's get_threading_mode/3 for every (n, workers) up to (40, 9);
   * the plan's batches, run through the oracle, give exactly the files the reference's own run writes (workers, same-seed workers, more
     workers than cases);
   * the parent state the engine's host code hands the device makes case I take the (I - A)-th seed of the worker's stream (checked
-    against the oracle's thread seeds through eb200_debug_parent_draws)."""
+    against the oracle's thread seeds through eb200_debug_parent_draws).
+The reference's side of the first two, executed from its source, is stored in tests/golden/reference_workers.json."""
 import ctypes as C
+import hashlib
+import json
 import os
-import sys
 
 import pytest
 
 import corpus
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, os.path.join(ROOT, "oracle"))
-HAVE_REF = os.path.exists("/root/reference/src/erlamsa_main.erl")
+HERE = os.path.dirname(os.path.abspath(__file__))
+PLANS = [(11, 3, (1, 2, 3), False), (12, 4, (4, 5, 6), False), (10, 3, (5, 1, 2), True), (5, 8, (3, 3, 3), False)]
+MUTS = {"bd": 1, "bf": 1, "num": 2, "ld": 1, "sr": 1, "fn": 1}
+PATS = {"od": 1, "nd": 1, "sk": 1}
+GENS = {"random": 1, "file": 1000}
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="needs the reference's sources (build container only)")
+def plan_files():
+    return [corpus.text_lines(corpus.rng(1200), 900), corpus.numeric_text(corpus.rng(1201), 500), corpus.random_bytes(corpus.rng(3), 700)]
+
+
+def plan_name(n, w, seed, same):
+    return "%d_%d_%d.%d.%d_%s" % ((n, w) + tuple(seed) + ("same" if same else "own",))
+
+
+def reference_answers():
+    """what the reference's own source answered (tests/golden/make_reference_workers.py)"""
+    with open(os.path.join(HERE, "golden", "reference_workers.json")) as f:
+        return json.load(f)
+
+
 def test_threading_mode_equals_the_reference_function():
-    from erlref.refrun import Reference
-    from erlref.terms import to_py, from_py
     from erlamsa_b200.workers import threading_mode
-    rt = Reference().rt
-    out = from_py([ord(c) for c in "out/%n"])
-    for n in range(1, 41):
-        for w in range(1, 10):
-            got = threading_mode("out/%n", n, w)
-            ref = rt.call("erlamsa_main", "get_threading_mode", out, n, w)
-            if ref == 1:
-                assert got is None, (n, w)
-                continue
-            ref = to_py(ref)
-            assert [((a, b, wn), r) for wn, (a, b, r) in enumerate(got)] == [((t[0][0], t[0][1], t[0][2]), t[1]) for t in ref], (n, w, got, ref)
+    modes = reference_answers()["threading_mode"]
+    assert len(modes) == 40 * 9
+    for n, w, ref in modes:
+        got = threading_mode("out/%n", n, w)
+        if ref is None:
+            assert got is None, (n, w)
+            continue
+        assert [[a, b, wn, r] for wn, (a, b, r) in enumerate(got)] == ref, (n, w, got, ref)
     assert threading_mode("return", 100, 4) is None and threading_mode("-", 100, 4) is None
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="needs the reference's sources (build container only)")
-@pytest.mark.parametrize("n,w,seed,same", [(11, 3, (1, 2, 3), False), (12, 4, (4, 5, 6), False), (10, 3, (5, 1, 2), True), (5, 8, (3, 3, 3), False)])
+@pytest.mark.parametrize("n,w,seed,same", PLANS)
 def test_plan_through_the_oracle_writes_the_reference_files(oracle, n, w, seed, same):
-    from erlref.refrun import Reference
-    from erlref.terms import from_py
     from erlamsa_b200.workers import worker_plan
-    sys.setrecursionlimit(3000000)
-    ref = Reference(budget=400_000_000)
-    rt = ref.rt
-    files = [corpus.text_lines(corpus.rng(1200), 900), corpus.numeric_text(corpus.rng(1201), 500), corpus.random_bytes(corpus.rng(3), 700)]
-    rt.vfs = {"f%d" % i: b for i, b in enumerate(files)}
-    muts = {"bd": 1, "bf": 1, "num": 2, "ld": 1, "sr": 1, "fn": 1}
-    pats = {"od": 1, "nd": 1, "sk": 1}
-    gens = {"random": 1, "file": 1000}
-    opts = ref.opts_map(b"", seed, muts, pats, n=n, skip=0, generators=gens)
-    del opts["input"]
-    opts["paths"] = from_py([from_py([ord(c) for c in p]) for p in ["f0", "f1", "f2"]])
-    opts["output"] = from_py([ord(c) for c in "out/%n"])
-    opts["workers"] = w
-    if same:
-        opts["workers_same_seed"] = "true"
-    opts["maxrunningtime"] = 600000
-    rt.vfs_out = {}
-    rt.steps = 0; rt.budget = ref.budget; rt.child_draws = []; rt.last_crash = None
-    rt.call("erlamsa_main", "fuzzer", opts)
-    written = dict(rt.vfs_out)
+    files = plan_files()
+    written = reference_answers()["plans"][plan_name(n, w, seed, same)]                 # file name -> [length, sha256] of what the reference wrote
     assert sorted(written) == sorted("out/%d" % i for i in range(1, n + 1))
     seen = set()
     for wseed, first, cnt, stream_first in worker_plan(seed, "out/%n", n, w, same):
-        outs, meta = oracle.fuzzer(files, mutations=muts, patterns=pats, seed=seed, generators=gens, n_cases=cnt, first_case=first, max_case_out=1 << 24,
+        outs, meta = oracle.fuzzer(files, mutations=MUTS, patterns=PATS, seed=seed, generators=GENS, n_cases=cnt, first_case=first, max_case_out=1 << 24,
                                    case_stream=(wseed, stream_first))
         for k in range(cnt):
-            assert meta[k].status == 0 and written["out/%d" % (first + k)] == outs[k], (first + k)
+            assert meta[k].status == 0 and written["out/%d" % (first + k)] == [len(outs[k]), hashlib.sha256(outs[k]).hexdigest()], (first + k)
             seen.add(first + k)
     assert seen == set(range(1, n + 1))
 
