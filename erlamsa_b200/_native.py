@@ -28,7 +28,7 @@ class Opts(C.Structure):
                 ("ssrf_host", C.c_char * 64), ("ssrf_port", C.c_int32), ("rng_mode", C.c_int32),
                 ("first_case", C.c_uint64), ("max_case_out", C.c_uint64), ("scratch_bytes", C.c_uint64),
                 ("donor_pool", C.c_void_p), ("donor_len", C.c_void_p), ("n_donors", C.c_uint64), ("donor_stride", C.c_uint32), ("reserved0", C.c_uint32),
-                ("gen_file_pri", C.c_int32), ("gen_stdin_pri", C.c_int32), ("gen_jump_pri", C.c_int32), ("reserved1", C.c_int32),
+                ("gen_file_pri", C.c_int32), ("gen_stdin_pri", C.c_int32), ("gen_jump_pri", C.c_int32), ("jump_on_device", C.c_int32),
                 ("case_stream_seed", C.c_int64 * 3), ("case_stream_first", C.c_uint64)]
 
 

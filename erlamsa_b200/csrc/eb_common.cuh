@@ -90,7 +90,7 @@ struct BatchParams {
     int32_t pat_sum;
     int32_t pat_pri[P_COUNT];
     int32_t pat_id[P_COUNT];
-    int32_t generator;             // 0 direct, 1 random
+    int32_t generator;             // 0 direct, 1 random, 2 file, 3 stdin, 4 jump
     int32_t rbs_bound;             // round(4096 * blockscale): bound of the unused rand_block_size draw
     int32_t rbs_min;               // round(256 * blockscale)
     uint64_t first_case;

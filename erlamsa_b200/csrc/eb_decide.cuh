@@ -2,7 +2,7 @@
 //
 // Mirrors, per case I (reference file:line):
 //   thread seed        erlamsa_main.erl:179-183   gen_predictable_seed on the parent stream (jump-ahead)
-//   generator          erlamsa_gen.erl:43-56,152-178   direct (+ finish tail) or random stream
+//   generator          erlamsa_gen.erl:43-178   direct (+ finish tail), random stream, file / stdin / jump streams (lazy)
 //   pattern            erlamsa_patterns.erl:266-443   od / nd / bu / sk / co / nu state machine
 //   scheduler          erlamsa_mutations.erl:1234-1280   weighted permutation, try until hd(Ll) changes
 // and leaves an edit script (list of Seg) + output length per case. No payload bytes are moved
@@ -187,14 +187,94 @@ EB_DEV const uint8_t* random_block_dev(CaseCtx& c, uint32_t n) {   // random_blo
     random_block_fill(c, buf, n);
     return buf;
 }
-// finish/1 :43-51 after `len` bytes of stream
-EB_DEV void finish_tail(CaseCtx& c, uint64_t len) {
-    WarpState* ws = c.ws; Rng& g = c.rng;
+// finish/1 :43-51 after `len` bytes of stream: true when it adds a random tail block (false: no tail, or the scratch arena is out)
+EB_DEV bool finish_block(CaseCtx& c, uint64_t len, Blk& tb) {
+    Rng& g = c.rng;
     uint64_t x = g.rand(len + 1);
-    if (x != len) return;
+    if (x != len) return false;
     uint64_t bits = (uint64_t)g.rand_range(1, 16);
     uint32_t nlen = (uint32_t)g.rand(1ull << bits);
-    if (nlen) { const uint8_t* t = random_block_dev(c, nlen); if (t) { Blk tb; tb.p = t; tb.len = nlen; tb.cnt = 1; runs_push_back(ws, tb); } }
+    if (!nlen) return false;
+    const uint8_t* t = random_block_dev(c, nlen);
+    if (!t) return false;
+    tb.p = t; tb.len = nlen; tb.cnt = 1;
+    return true;
+}
+EB_DEV void finish_tail(CaseCtx& c, uint64_t len) {
+    Blk tb;
+    if (finish_block(c, len, tb)) runs_push_back(c.ws, tb);
+}
+// ------------------------------------------------------------------ jump generator (reference src/erlamsa_gen.erl:123-150)
+// Block cutter of stream_port/5 over n bytes, 32 rand_block_size draws per step: lane l evaluates draw `done + l` of the stream
+// (AS183: its own state x * a^(done + l), stepped by a^32; Philox: uniform_philox_at), an inclusive scan says where each block
+// ends, and the first lane whose block does not fit ends the stream. It draws from a COPY of `g`: `draws` (full blocks + 1, the
+// same draws as the serial loop) is how far the caller's stream has to advance. With want < nfull the walk stops at block
+// `want` and returns its place (the replay that finds a picked block without keeping the block list anywhere).
+struct JumpCut { uint32_t nfull, pos; uint64_t draws; uint32_t at, len; };
+EB_DEV JumpCut jump_cut(const Rng& g, const BatchParams* bp, uint32_t n, uint32_t want) {
+    const int l = lane_id();
+    JumpCut r; r.nfull = 0; r.pos = 0; r.draws = 0; r.at = 0; r.len = 0;
+    Rng mine = g;
+    if (g.mode == 0) mine.jump((uint64_t)l);
+    const uint32_t s1 = modpow_u32<30269>(AS_M1, 31), s2 = modpow_u32<30307>(AS_M2, 31), s3 = modpow_u32<30323>(AS_M3, 31);
+    for (;;) {
+        double u;
+        if (g.mode == 0) {
+            u = mine.uniform_as183();
+            mine.a1 = (int32_t)(((uint32_t)mine.a1 * s1) % 30269u); mine.a2 = (int32_t)(((uint32_t)mine.a2 * s2) % 30307u); mine.a3 = (int32_t)(((uint32_t)mine.a3 * s3) % 30323u);
+        } else u = g.uniform_philox_at(g.local + (uint32_t)r.draws + (uint32_t)l);
+        uint64_t x = (uint64_t)trunc(u * (double)bp->rbs_bound);                 // rand(rbs_bound)
+        uint64_t w = x > (uint64_t)bp->rbs_min ? x : (uint64_t)bp->rbs_min;      // rand_block_size :55-56
+        uint64_t end = w;
+        for (int o = 1; o < 32; o <<= 1) { uint64_t y = __shfl_up_sync(0xffffffffu, end, o); if (l >= o) end += y; }
+        unsigned miss = __ballot_sync(0xffffffffu, (uint64_t)r.pos + end > (uint64_t)n);
+        uint32_t nfit = miss ? (uint32_t)(__ffs(miss) - 1) : 32u;
+        if (want < r.nfull + nfit) {
+            int j = (int)(want - r.nfull);
+            uint64_t e = __shfl_sync(0xffffffffu, end, j), wj = __shfl_sync(0xffffffffu, w, j);
+            r.at = r.pos + (uint32_t)(e - wj); r.len = (uint32_t)wj;
+            return r;
+        }
+        if (nfit) r.pos += (uint32_t)__shfl_sync(0xffffffffu, end, (int)nfit - 1);
+        r.nfull += nfit;
+        if (miss) { r.draws += nfit + 1; return r; }
+        r.draws += 32;
+    }
+}
+// one file of jump_somewhere/2: the whole stream (every block-size draw, then finish/1), then erand over its blocks.
+// false: the case ends here (an empty block list: the worker dies; or the scratch arena is out)
+EB_DEV bool jump_pick(CaseCtx& c, const uint8_t* p, uint32_t n, const uint8_t*& d, uint32_t& dn) {
+    WarpState* ws = c.ws; Rng& g = c.rng;
+    const Rng saved = g;
+    JumpCut cut = jump_cut(g, c.bp, n, 0xffffffffu);
+    if (g.mode == 0) g.jump(cut.draws); else g.philox_skip((uint32_t)cut.draws);
+    uint32_t rest = n - cut.pos;
+    Blk tail; bool has_tail = finish_block(c, n, tail);
+    if (ws->status != CASE_OK) return false;
+    uint64_t nb = (uint64_t)cut.nfull + (rest ? 1 : 0) + (has_tail ? 1 : 0);
+    if (nb == 0) { ws->status = CASE_DIED; return false; }   // rand_elem([]) is [], size([]) raises
+    uint64_t k = g.erand(nb) - 1;
+    if (k < cut.nfull) { JumpCut b = jump_cut(saved, c.bp, n, (uint32_t)k); d = p + b.at; dn = b.len; }
+    else if (k == cut.nfull && rest) { d = p + cut.pos; dn = rest; }
+    else { d = tail.p; dn = tail.len; }
+    return true;
+}
+// jump_somewhere/2 :123-132: a block of each file, then S1, S2, L1, L2; the block list becomes the one block
+// Data1[S1, S1+L1) ++ Data2[S2, S2+L2), materialised in scratch
+EB_DEV void force_jump(CaseCtx& c) {
+    WarpState* ws = c.ws; Rng& g = c.rng;
+    // blockscale < 1/512: rand_block_size can be 0, and a zero-size block never ends the stream (the reference loops)
+    if (c.bp->rbs_min == 0) { ws->status = CASE_UNSUPPORTED; ws->reason = 12; return; }
+    const uint8_t *d1, *d2; uint32_t n1, n2;
+    if (!jump_pick(c, ws->lz_p, ws->lz_n, d1, n1)) return;
+    if (!jump_pick(c, ws->lz_p2, ws->lz_n2, d2, n2)) return;
+    uint64_t s1 = g.rand(n1), s2 = g.rand(n2);
+    uint64_t l1 = g.erand(n1 - s1), l2 = g.erand(n2 - s2);
+    uint8_t* buf = scratch_alloc(c, l1 + l2);
+    if (!buf) return;
+    warp_copy(buf, d1 + s1, l1); warp_copy(buf + l1, d2 + s2, l2);
+    __syncwarp();
+    Blk b; b.p = buf; b.len = (uint32_t)(l1 + l2); b.cnt = 1; runs_push_back(ws, b);
 }
 // file / stdin generators (reference src/erlamsa_gen.erl:59-121): port_stream/2 returns an UNFORCED stream, so the blocks
 // (stream_port/5: full blocks of the wanted size, a new rand_block_size after each, the short rest last) and the finish/1
@@ -203,6 +283,7 @@ EB_DEV void force_stream(CaseCtx& c) {
     WarpState* ws = c.ws; Rng& g = c.rng; const BatchParams* bp = c.bp;
     if (!ws->lazy) return;
     ws->lazy = 0;
+    if (bp->generator == 4) { force_jump(c); return; }
     const uint8_t* p = ws->lz_p; uint32_t n = ws->lz_n, pos = 0;
     uint64_t r0 = g.rand((uint64_t)bp->rbs_bound);
     uint32_t wanted = (uint32_t)(r0 > (uint64_t)bp->rbs_min ? r0 : (uint64_t)bp->rbs_min);
@@ -228,6 +309,13 @@ EB_DEV void generate(CaseCtx& c, const uint8_t* blob, uint32_t blen, const uint8
             blob = data + off[pi]; blen = (uint32_t)(off[pi + 1] - off[pi]);
         }
         ws->lazy = 1; ws->lz_p = blob; ws->lz_n = blen;
+        return;
+    }
+    if (bp->generator == 4) {       // jump_streamer :135-150: P1, P2 = erand(N) now, the block at the first uncons
+        uint64_t p1 = g.erand(bp->n_blobs) - 1, p2 = g.erand(bp->n_blobs) - 1;
+        ws->lazy = 1;
+        ws->lz_p = data + off[p1]; ws->lz_n = (uint32_t)(off[p1 + 1] - off[p1]);
+        ws->lz_p2 = data + off[p2]; ws->lz_n2 = (uint32_t)(off[p2 + 1] - off[p2]);
         return;
     }
     if (bp->generator == 0) {   // direct_generator + finish
@@ -485,10 +573,12 @@ struct FusedArgs { int fused; uint8_t* out; uint64_t out_capacity; const uint64_
                    const uint32_t* case_list; uint64_t n_list; unsigned long long* case_counter; int deciders; int fronts; int front_depth; int tma_workers; };
 
 // slot sizes for the single-pass mode: input length + slack, 16-byte aligned (the common mutations change a
-// case by a few bytes; anything bigger spills to the overflow region)
-__global__ void __launch_bounds__(256) eb_slot_sizes(const uint64_t* __restrict__ off, uint64_t first_case, uint64_t n_blobs, uint64_t n_cases, uint64_t* __restrict__ sz16) {
+// case by a few bytes; anything bigger spills to the overflow region). fixed != 0: every slot has that size (the jump
+// generator, whose result is a slice of two blocks and has nothing to do with blob (I-1) mod n)
+__global__ void __launch_bounds__(256) eb_slot_sizes(const uint64_t* __restrict__ off, uint64_t first_case, uint64_t n_blobs, uint64_t n_cases, uint64_t fixed, uint64_t* __restrict__ sz16) {
     uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= n_cases) return;
+    if (fixed) { sz16[k] = fixed; return; }
     uint64_t b = (first_case - 1 + k) % n_blobs;
     uint64_t len = off[b + 1] - off[b];
     uint64_t slack = len / 16; if (slack < 256) slack = 256; if (slack > 65536) slack = 65536;
@@ -539,7 +629,8 @@ EB_DEV void decide_one_case(WarpState* ws, const BatchParams& bp, const DecideAr
             if (FULL && ws->status == CASE_OK) unwind_wrappers(c);
         }
         if (ws->status == CASE_OK && ws->olen > bp.max_case_out) { ws->status = CASE_OVERFLOW; ws->reason = 5; }
-        if (ws->status == CASE_UNSUPPORTED || ws->status == CASE_OVERFLOW) { ws->noseg = 0; ws->olen = 0; o_push(c, seg_copy(blob, blen)); }
+        // a flagged case outputs its input unchanged -- except under jump, whose slots are not sized from the input: nothing
+        if (ws->status == CASE_UNSUPPORTED || ws->status == CASE_OVERFLOW) { ws->noseg = 0; ws->olen = 0; if (bp.generator != 4) o_push(c, seg_copy(blob, blen)); }
         if (ws->status == CASE_DIED) { ws->noseg = 0; ws->olen = 0; }
         __syncwarp();
         unsigned long long sb = 0; int ns = ws->noseg;
@@ -562,9 +653,9 @@ EB_DEV void decide_one_case(WarpState* ws, const BatchParams& bp, const DecideAr
                     }
                 }
                 o = __shfl_sync(0xffffffffu, o, 0);
-                if (o == ~0ull) {   // no room: flag the case, emit the input unchanged (always fits its slot)
+                if (o == ~0ull) {   // no room: flag the case, emit the input unchanged (always fits its slot; jump: nothing)
                     if (lane_id() == 0) atomicOr(ar.overflow, 4u);
-                    ws->status = CASE_OVERFLOW; ws->reason = 11; ws->noseg = 0; ws->olen = 0; o_push(c, seg_copy(blob, blen)); ns = ws->noseg;
+                    ws->status = CASE_OVERFLOW; ws->reason = 11; ws->noseg = 0; ws->olen = 0; if (bp.generator != 4) o_push(c, seg_copy(blob, blen)); ns = ws->noseg;
                 } else dsto = a.ovf_base + o;
             }
             segs_write_stream(q, ws->oseg, ws->noseg, a.out + dsto, data, data + a.data_bytes);

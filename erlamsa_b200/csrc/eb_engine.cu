@@ -168,7 +168,7 @@ static int compute_batch_params(const eb200_opts* o, uint64_t n_blobs, uint64_t 
     if (gs.empty()) return EB200_ERR_ARG;
     { auto sg = sort_by_priority(gs); int sum = 0; for (auto& g : sg) sum += g.first;
       int g = choose_pri(sg, (int64_t)par.rand((uint64_t)sum)); if (g < 0) return EB200_ERR_ARG; bp.generator = g;
-      if (g == 4) return EB200_ERR_UNSUPPORTED; }                        // the draw is the reference's; the jump generator itself is not on the device
+      if (g == 4 && !o->jump_on_device) return EB200_ERR_UNSUPPORTED; }  // the draw is the reference's; running jump is opt-in
     std::vector<std::pair<int, int>> ps;                                 // make_pattern: foldl prepends -> reversed table
     for (int i = P_COUNT - 1; i >= 0; i--) if (o->pat_pri[i] >= 0) {
         if (o->pat_pri[i] > 0 && !pat_supported(i)) return EB200_ERR_UNSUPPORTED;
@@ -342,6 +342,20 @@ static void launch_cases(eb200_ctx* ctx, const BatchParams& bp, const LaunchPlan
     else eb_case_kernel<false><<<lp.grid, lp.threads, sm, st>>>(d_data, d_off, bp, lp.ar, (CaseOut*)ctx->cases.p, d_out_len, (uint64_t*)ctx->sz16.p, (MetaDev*)d_meta, fa);
 }
 
+// Output slot of every case of a jump batch: the result is a slice of one block of each file (blocks are below rbs_bound, a finish/1
+// tail below 64 KiB), mostly well under one block, so the slot is what eb_slot_sizes gives an input of rbs_bound bytes; a bigger
+// result goes to the overflow region like any other.
+static uint64_t jump_slot_bytes(const BatchParams& bp) {
+    uint64_t len = (uint64_t)bp.rbs_bound;
+    return align16(len + std::min<uint64_t>(std::max<uint64_t>(len / 16, 256), 65536));
+}
+// scratch a batch wants up front: four times its input for the mutators' rounds, plus (jump) every case's result block
+static uint64_t scratch_bytes_for(const BatchParams& bp, const eb200_opts* opts, uint64_t data_bytes) {
+    if (opts->scratch_bytes) return opts->scratch_bytes;
+    uint64_t jump = bp.generator == 4 ? bp.n_cases * ((uint64_t)bp.rbs_bound + 32) : 0;
+    return std::min<uint64_t>(4 * data_bytes + jump + (64ull << 20), 8ull << 30);
+}
+
 // decide + scan for a batch resident on the device (two-pass mode). On return *total_out = packed output size.
 static int run_decide_scan(eb200_ctx* ctx, const BatchParams& bp, const eb200_opts* opts, const uint8_t* d_data, const uint64_t* d_off,
                            uint64_t data_bytes, uint64_t* d_out_off, uint64_t* d_out_len, eb200_meta* d_meta, cudaStream_t st, uint64_t* total_out, uint32_t* launches) {
@@ -354,7 +368,7 @@ static int run_decide_scan(eb200_ctx* ctx, const BatchParams& bp, const eb200_op
     CK(ctx->counters.ensure(64));
     uint64_t seg_cap = ctx->segs.cap / sizeof(Seg);
     if (seg_cap < n * 6 + 1024) { CK(ctx->segs.ensure((n * 6 + 1024) * sizeof(Seg))); seg_cap = ctx->segs.cap / sizeof(Seg); }
-    uint64_t scratch_want = opts->scratch_bytes ? opts->scratch_bytes : std::min<uint64_t>(4 * data_bytes + (64ull << 20), 8ull << 30);
+    uint64_t scratch_want = scratch_bytes_for(bp, opts, data_bytes);
     if (ctx->scratch.cap < scratch_want) CK(ctx->scratch.ensure(scratch_want));
     // edit scripts published by this mode point into scratch, so an exhausted arena means running the batch again
     for (int attempt = 0;; attempt++) {
@@ -416,10 +430,11 @@ static int run_fused(eb200_ctx* ctx, const BatchParams& bp, const eb200_opts* op
     CK(ctx->slot_off.ensure((n + 1) * 8));
     CK(ctx->counters.ensure(64));
     CK(ctx->cases.ensure(sizeof(CaseOut)));
-    uint64_t scratch_want = opts->scratch_bytes ? opts->scratch_bytes : std::min<uint64_t>(4 * data_bytes + (64ull << 20), 8ull << 30);
+    uint64_t scratch_want = scratch_bytes_for(bp, opts, data_bytes);
     if (ctx->scratch.cap < scratch_want) CK(ctx->scratch.ensure(scratch_want));
     CK(cudaEventRecord(ctx->ev[1], st));
-    eb_slot_sizes<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_off, bp.first_case, bp.n_blobs, n, (uint64_t*)ctx->sz16.p);
+    eb_slot_sizes<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_off, bp.first_case, bp.n_blobs, n, bp.generator == 4 ? jump_slot_bytes(bp) : 0,
+                                                               (uint64_t*)ctx->sz16.p);
     eb_scan_tiles<<<(unsigned)ntiles, SCAN_THREADS, 0, st>>>((const uint64_t*)ctx->sz16.p, n, (uint64_t*)ctx->tile_sum.p);
     eb_scan_tile_offsets<<<1, SCAN_THREADS, 0, st>>>((uint64_t*)ctx->tile_sum.p, ntiles, (uint64_t*)ctx->tile_sum.p + ntiles);
     eb_scan_finish<<<(unsigned)ntiles, SCAN_THREADS, 0, st>>>((const uint64_t*)ctx->sz16.p, n, (const uint64_t*)ctx->tile_sum.p, (const uint64_t*)ctx->tile_sum.p + ntiles, (uint64_t*)ctx->slot_off.p);
@@ -676,14 +691,18 @@ int eb200_fuzz_batch_into(eb200_ctx* ctx, const eb200_opts* opts, const uint8_t*
                           uint8_t* out_buf, uint64_t out_capacity, uint64_t* out_off, uint64_t* out_len, eb200_meta* meta, eb200_stats* stats) {
     if (!out_buf) return EB200_ERR_ARG;
     if (ctx && opts && off && data && out_off && out_len && n_blobs) {
-        // big batches whose cases read a contiguous run of blobs go through the overlapped pipeline
+        // big batches whose cases read a contiguous run of blobs go through the overlapped pipeline. It uploads each chunk's
+        // own blobs only, so it is for generators that read blob (I-1) mod n (direct, random, stdin): a file or jump case reads
+        // any blob. The generator draw is the parent's, host-only and cheap.
         uint64_t data_bytes = off[n_blobs];
         uint64_t first = opts->first_case ? opts->first_case : 1;
         uint64_t b0 = (first - 1) % n_blobs;
         bool ok = true;
         for (uint64_t b = 0; b < n_blobs && ok; b++) ok = off[b + 1] >= off[b] && off[b + 1] - off[b] <= 0xfffffff0ull;
         if (!ok) return EB200_ERR_ARG;
-        if (b0 + n_cases <= n_blobs && data_bytes >= (256ull << 20) && n_cases >= 4096) {
+        BatchParams bp;
+        bool own_blob = compute_batch_params(opts, n_blobs, n_cases, bp) == EB200_OK && bp.generator != 2 && bp.generator != 4;
+        if (own_blob && b0 + n_cases <= n_blobs && data_bytes >= (256ull << 20) && n_cases >= 4096) {
             uint64_t avg = std::max<uint64_t>(1, data_bytes / n_blobs);
             uint64_t chunk = std::max<uint64_t>(1024, ((uint64_t)ctx->chunk_mb << 20) / avg);
             if (chunk * 2 <= n_cases) return fuzz_batch_host_pipelined(ctx, opts, data, off, n_blobs, n_cases, out_buf, out_capacity, out_off, out_len, meta, stats, chunk);

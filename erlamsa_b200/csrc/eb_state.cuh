@@ -63,8 +63,10 @@ struct WarpState {
     struct Wrap { uint32_t kind; uint32_t bits; uint32_t big; uint32_t tail_n; uint64_t field_pos; uint64_t mark; const uint8_t* tail_p; } wrap[8];
     int nwrap;
     const uint8_t* fo_p; uint32_t fo_n; int fo_has;
-    // file / stdin generators: the block list does not exist until the pattern's first uncons (eb_decide.cuh force_stream)
+    // file / stdin / jump generators: the block list does not exist until the pattern's first uncons (eb_decide.cuh force_stream);
+    // jump keeps its second file in lz_p2 / lz_n2
     int lazy; const uint8_t* lz_p; uint32_t lz_n;
+    const uint8_t* lz_p2; uint32_t lz_n2;
     uint32_t round;          // mux_fuzzers rounds so far in this case (Philox counter slots, eb_rng.cuh)
     uint64_t donor;          // this case's donor index (thread seed hash, see mut_fuse)
     uint16_t sc[SC_MAX];

@@ -4,7 +4,9 @@ CUDA engine, for the generators and outputs that are part of the hot path's surr
     paths  => [direct] with input => Bin | [Bin]   direct generator (src/erlamsa_gen.erl:152-164); a LIST is a corpus: case I
                                                      mutates element (I-1) rem length -- the batched generalisation
     paths  => ["file1", "dir/file2", ...]           file generator (:104-121): every case picks one of the files (erand), which is
-                                                     cut lazily into random-size blocks (rand_block_size :55-56)
+                                                     cut lazily into random-size blocks (rand_block_size :55-56); with two or more
+                                                     files the parent's draw may land on jump (:123-150): a slice of a block of one
+                                                     file ++ a slice of a block of another
     paths  => ["-"]                                 stdin generator (:92-102), n == 1 only (the reference pre-reads stdin in the
                                                      parent process for n > 1, which is not modelled)
     output => return                                -> [binary()], empty results dropped like record_result/2 (:120-122)
@@ -70,9 +72,10 @@ def fuzzer(opts):
         n = int(opts.get("n", 1))
         if "generators" not in o:
             # what make_generator keeps of erlamsa_gen:default/0 for file paths (src/erlamsa_gen.erl:204-237): jump only with two or
-            # more paths. jump takes part in the parent's generator draw as in the reference; a run whose draw lands on it (100 in
-            # 1101) is refused by the engine (EngineError: no device implementation) instead of silently becoming another run.
+            # more paths. jump takes part in the parent's generator draw as in the reference (100 in 1101 runs land on it)
             o["generators"] = {"random": 1, "jump": 100, "file": 1000} if len(paths) > 1 else {"random": 1, "file": 1000}
+        if len(paths) > 1:
+            o.setdefault("jump_on_device", True)      # a run whose draw lands on jump runs it on the device
     plan = worker_plan(opts["seed"], output, n, int(opts.get("workers", 1)), bool(opts.get("workers_same_seed", False))) 
     for k in ("paths", "output", "input", "n", "skip", "stdin_data", "workers", "workers_same_seed"):
         o.pop(k, None)

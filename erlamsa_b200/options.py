@@ -105,10 +105,12 @@ def make_opts(opts=None):
         o.gen_random_pri = int(g.get("random", -1))
         o.gen_file_pri = int(g.get("file", -1))
         o.gen_stdin_pri = int(g.get("stdin", -1))
-        o.gen_jump_pri = int(g.get("jump", -1))      # takes part in the parent's draw; a run that lands on it is refused by the engine
+        o.gen_jump_pri = int(g.get("jump", -1))      # takes part in the parent's draw; a run that lands on it needs jump_on_device
         unknown = set(g) - {"direct", "random", "file", "stdin", "jump"}
         if unknown:
             raise ValueError("generator(s) without a device implementation: %s" % ", ".join(sorted(unknown)))
+    # 1: run the jump generator when the parent's draw lands on it; 0 (default): the engine refuses such a run (EB200_ERR_UNSUPPORTED)
+    o.jump_on_device = 1 if opts.get("jump_on_device") else 0
     if opts.get("case_stream") is not None:       # (worker seed, number of the worker's first case): one worker of `workers` > 1
         (a, b, c), first = opts["case_stream"]
         o.case_stream_seed[0], o.case_stream_seed[1], o.case_stream_seed[2] = int(a), int(b), int(c)

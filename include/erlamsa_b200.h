@@ -55,6 +55,9 @@ extern "C" {
                                         the `ar` pattern as continuation); output = input unchanged */
 #define EB200_CASE_DIED          2   /* the reference's worker process would have crashed; output empty */
 #define EB200_CASE_OVERFLOW      3   /* out of scratch, output cap or descriptor space; output = input unchanged */
+/* Under the jump generator a flagged case (UNSUPPORTED or OVERFLOW) outputs NOTHING: its slot is sized from the block size, not
+ * from an input, so "the input unchanged" need not fit it. status / reason say why. Reason 12 (jump only): blockscale < 1/512
+ * makes rand_block_size 0 possible, and a zero-size block never ends the file's stream (the reference loops forever). */
 
 typedef struct eb200_ctx eb200_ctx;
 
@@ -92,10 +95,12 @@ typedef struct eb200_opts {
     int32_t  gen_file_pri;
     int32_t  gen_stdin_pri;
     /* `jump` (100; src/erlamsa_gen.erl:123-150, kept by make_generator only when there are two or more paths): it takes part in the
-     * parent's generator draw exactly as in the reference (rand over the priority sum, :194-199), so that a run whose draw lands on
-     * file / random is the reference's run; a run whose draw lands on jump has no device implementation: EB200_ERR_UNSUPPORTED. */
+     * parent's generator draw exactly as in the reference (rand over the priority sum, :194-199). A run whose draw lands on jump is
+     * run on the device when jump_on_device is 1: every case picks two blobs (erand(n_blobs) twice), cuts each into random-size
+     * blocks, picks one block of each and outputs the mutation of a random slice of the first ++ a random slice of the second.
+     * With jump_on_device 0 (the default) such a run is refused with EB200_ERR_UNSUPPORTED, so that a caller can route it elsewhere. */
     int32_t  gen_jump_pri;
-    int32_t  reserved1;
+    int32_t  jump_on_device;                /* 1: run the jump generator when the draw lands on it; 0: EB200_ERR_UNSUPPORTED */
     /* Multi-threaded mode of the reference (option `workers` > 1 with a file / network output, run_fuzzing_loop/7, src/erlamsa_main.erl:
      * 254-280): every worker process is re-seeded with its own seed S (the W-th gen_predictable_seed() of the re-seeded parent, or the
      * run's seed with `workers_same_seed`) and draws the thread seed of ITS first case, number A, as the first three draws of that
@@ -108,13 +113,14 @@ typedef struct eb200_opts {
 
 typedef struct eb200_meta {
     int32_t  pattern;        /* first pattern chosen (index into the pattern table) */
-    int32_t  generator;      /* 0 direct, 1 random */
+    int32_t  generator;      /* 0 direct, 1 random, 2 file, 3 stdin, 4 jump */
     int32_t  n_used;         /* successful mutator applications */
     int32_t  n_failed;       /* attempts that left hd(Ll) unchanged */
     int32_t  used[16];       /* first 16 used mutator ids (table index), -1 padded */
     uint64_t draws;          /* RNG draws consumed by the case's worker stream */
     int32_t  status;         /* EB200_CASE_* */
-    int32_t  reason;         /* why a case was flagged (DESIGN.md section 6): 1 scratch, 4 block runs, 5 output cap, 8 fuse tables, 11 output arena, ... */
+    int32_t  reason;         /* why a case was flagged (DESIGN.md section 6): 1 scratch, 4 block runs, 5 output cap, 8 fuse tables, 11 output arena,
+                                12 jump with a zero block size, ... */
     int64_t  thread_seed[3]; /* the case's erlamsa_rnd:gen_predictable_seed() */
 } eb200_meta;
 
@@ -145,7 +151,8 @@ void eb200_shutdown(eb200_ctx* ctx);
  *   out_off  : caller array of n_cases+1 entries: case k output = (*out_data)[out_off[k] .. out_off[k]+out_len[k]);
  *              out_off[n_cases] = bytes used in the buffer. Case regions are 16-byte aligned and do not overlap, but
  *              they are NOT back to back: in the default single-pass mode each case owns a slot sized from its input
- *              (plus slack) and larger results live behind the slots, so always go through out_off / out_len.
+ *              (plus slack; under jump from the block size) and larger results live behind the slots, so always go through
+ *              out_off / out_len.
  *   out_len  : caller array of n_cases entries
  *   meta     : optional caller array of n_cases entries
  */
@@ -221,7 +228,7 @@ int  eb200_async_lanes(eb200_ctx* ctx);        /* lanes created so far (0 before
  * restates before it launches anything (src/erlamsa_main.erl:127-163; SURVEY.md appendix A, T0..T3). out[0] = generator chosen
  * (0 direct, 1 random, 2 file, 3 stdin, 4 jump), out[1] = snand mask kind, out[2] = table rows, out[3] = patterns, out[4..6] = the
  * parent's AS183 state after its draws (the first case's thread seed is the next three erand(99999)). Returns what the batch call
- * would return for these options (EB200_ERR_UNSUPPORTED when the draw lands on jump). */
+ * would return for these options (EB200_ERR_UNSUPPORTED when the draw lands on jump and jump_on_device is 0). */
 int eb200_debug_parent_draws(const eb200_opts* opts, uint64_t n_blobs, uint64_t n_cases, int64_t out[8]);
 
 /* name surface of the reference (-m / -p codes, src/erlamsa_cmdparse.erl:233-257) */
